@@ -5,6 +5,7 @@
     python bench.py --impl reference [...]                                       # UNMODIFIED reference on host cores
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...             # one rank per GPU (weak scaling)
     python bench.py --model vit_l16|vit_h14|navit [--dim-head 80]                # the other BASELINE.json configs
+    python bench.py --dump-outputs DIR [...]     # also write the logits of the last timed step to DIR/logits.npy
 
 One "step" = one forward of a synthetic batch per GPU (+ the all-gather of the logits when N > 1).  Prints ONE JSON
 line on rank 0 (see DESIGN.md "Measurement" for every field).
@@ -14,6 +15,8 @@ Baselines carried by the GPU arm's line (rank 0, N = 1):
   * `gpu_eager_baseline`  the unmodified reference's eager bf16 forward on the SAME GPU, same weights, same batch,
                           same CUDA-event protocol (the on-box bar of BASELINE.md section 5), plus the max |logit|
                           difference between it and the fused path.
+Both legs need the unmodified reference installed under baseline/_ref/, which is not part of the repository: without
+it `gpu_eager_baseline` reports "unavailable" and `cpu_baseline` times the oracle port instead (kind "port").
 """
 from __future__ import annotations
 
@@ -24,8 +27,12 @@ import random
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it
+
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -104,17 +111,20 @@ class ClockSampler:
     def __init__(self, index: int) -> None:
         self.index = index
         self.proc = None
-        self.path = os.path.join(ROOT, "gpurun_out", f"clocks_{index}.csv")
+        self.path = None
 
     def start(self) -> None:
         try:
-            os.makedirs(os.path.dirname(self.path), exist_ok=True)
-            self.f = open(self.path, "w")
+            fd, self.path = tempfile.mkstemp(prefix=f"b200vit_clocks_{self.index}_", suffix=".csv")
+            self.f = os.fdopen(fd, "w")
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.index), f"--query-gpu={self.FIELDS}",
                                           "--format=csv,noheader,nounits", "-lms", "100"], stdout=self.f,
                                          stderr=subprocess.DEVNULL)
         except Exception:
             self.proc = None
+            if self.path:
+                self.f.close()
+                os.unlink(self.path)
 
     def stop(self) -> dict:
         if self.proc is None:
@@ -127,7 +137,10 @@ class ClockSampler:
         self.f.close()
         sm, mx, pw, reasons = [], [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
-        for line in open(self.path):
+        with open(self.path) as f:
+            lines = f.readlines()
+        os.unlink(self.path)
+        for line in lines:
             parts = [x.strip() for x in line.split(",")]
             if len(parts) < 7:
                 continue
@@ -382,21 +395,26 @@ def run_gpu_arm(args, rank: int, local_rank: int, world: int) -> None:
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-        time.sleep(0.3)
-    _lib.reset_launch_count()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    sync_all()
-    e0.record()
-    for _ in range(args.steps):
-        out = step(img)
-    e1.record()
-    torch.cuda.synchronize()
-    launches = _lib.launch_count()
-    per_rank_ms = all_ranks(e0.elapsed_time(e1))
-    ms_total = max(per_rank_ms)
-    sync_all()
-    clocks = sampler.stop() if sampler else None
+    try:                                         # the nvidia-smi sampler never outlives the timed region
+        if sampler:
+            time.sleep(0.3)
+        _lib.reset_launch_count()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        sync_all()
+        e0.record()
+        for _ in range(args.steps):
+            out = step(img)
+        e1.record()
+        torch.cuda.synchronize()
+        launches = _lib.launch_count()
+        per_rank_ms = all_ranks(e0.elapsed_time(e1))
+        ms_total = max(per_rank_ms)
+        sync_all()
+    finally:
+        clocks = sampler.stop() if sampler else None
     value = world * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:         # outside the sampled window; `out` is still the last timed step's
+        dump_outputs(args.dump_outputs, {"logits": out})
 
     # ---- per-rank compute without the collective (N > 1): which GPU sets the pace of the coupled step ----
     per_rank_compute_ms = None
@@ -585,6 +603,23 @@ def run_gpu_arm(args, rank: int, local_rank: int, world: int) -> None:
         dist.destroy_process_group()
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Each array as float32 `directory/<name>.npy`.  An array larger than its share of DUMP_BYTES keeps a fixed,
+    seeded sample of its rows (in order), so that two builds can be compared output for output."""
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        row_bytes = a[0].numel() * 4 if a.dim() > 1 else 4
+        if a.numel() * 4 > share:
+            keep = max(1, share // row_bytes)
+            rows = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            a = a[rows]
+        np.save(os.path.join(directory, name + ".npy"), a.numpy())
+
+
 def gpu_eager_baseline(args, CFG, model, img, our_out, dev, B):
     """Reference eager bf16 forward on this GPU (cuBLASLt + ATen kernels, what a user of the reference gets today)."""
     ref = build_reference_model(args.model, CFG)
@@ -636,7 +671,20 @@ def main() -> None:
                     help="reference arm: seconds the timed steps may take; the per-step sample is halved until they fit")
     ap.add_argument("--model", default="vit_b16", choices=sorted(MODELS), help="vit_b16 is the headline config")
     ap.add_argument("--dim-head", type=int, default=64, help="ViT-H/14 canonical is 80")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits of the last timed step to DIR/logits.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "b200":
+            ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+        try:                                     # fail before any GPU work, not after the timed steps
+            os.makedirs(args.dump_outputs, exist_ok=True)
+        except OSError as e:
+            ap.error(f"--dump-outputs {args.dump_outputs}: {e}")
+        if not os.access(args.dump_outputs, os.W_OK | os.X_OK):
+            ap.error(f"--dump-outputs {args.dump_outputs}: directory is not writable")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

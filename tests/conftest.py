@@ -10,11 +10,11 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+if GOLDEN_DIR not in sys.path:
+    sys.path.insert(0, GOLDEN_DIR)
+from golden_weights import load, state_digest  # noqa: E402,F401  (tests/golden/)
+
 GOLDEN_NAMES = ["simplevit_tiny", "vit_tiny_cls", "vit_tiny_mean_nonsquare", "vit_tiny_tokens"]
-REFERENCE_DIR = os.environ.get("VIT_REFERENCE", "/root/reference")
-if not os.path.isdir(os.path.join(REFERENCE_DIR, "vit_pytorch")):
-    # GPU box: the unmodified reference installed under baseline/_ref travels with the snapshot (DESIGN.md 8)
-    REFERENCE_DIR = os.path.join(ROOT, "baseline", "_ref")
 
 
 def pytest_configure(config):
@@ -31,7 +31,7 @@ def pytest_collection_modifyitems(config, items):
 
 
 def load_golden(name):
-    return torch.load(os.path.join(GOLDEN_DIR, name + ".pt"), weights_only=False)
+    return load(os.path.join(GOLDEN_DIR, name + ".pt"))
 
 
 @pytest.fixture(params=GOLDEN_NAMES)
@@ -39,14 +39,11 @@ def golden(request):
     return load_golden(request.param)
 
 
-def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_DIR, "vit_pytorch"))
-
-
-def import_reference():
-    """Import the unmodified reference package (build container only)."""
-    import importlib
-    sys.dont_write_bytecode = True
-    if REFERENCE_DIR not in sys.path:
-        sys.path.insert(0, REFERENCE_DIR)
-    return importlib.import_module("vit_pytorch")
+def reference_init(name: str, cls):
+    """`cls` built under the seed and keywords of reference_surface.pt's `init[name]`, after checking that it draws
+    bit-identical parameters to the reference's constructor (key order, shapes, values)."""
+    spec = load_golden("reference_surface")["init"][name]
+    torch.manual_seed(spec["seed"])
+    m = cls(**spec["kwargs"])
+    assert list(state_digest(m.state_dict()).items()) == list(spec["digest"].items()), name
+    return m

@@ -7,8 +7,9 @@ Run in the build container only (the GPU box has no /root/reference):
 For each case: build the reference model under torch.manual_seed(seed), round its parameters to bf16-representable
 values (so the same numbers can be fed to the bf16 CUDA path), run the reference forward in fp32 on CPU on a
 bf16-representable input, and additionally run the reference's own bf16 forward (its noise floor).  Saved per case
-(tests/golden/<name>.pt): kind, ctor kwargs, state_dict (bf16), input (bf16), logits_fp32, logits_ref_bf16,
-tokens_fp32 (transformer output for the first sample) and the library versions.
+(tests/golden/<name>.pt): kind, ctor kwargs, seed and the sha256 digest of the bf16 state_dict (golden_weights.py
+rebuilds the weights from the seed), input (bf16), logits_fp32, logits_ref_bf16, tokens_fp32 (transformer output for
+the first sample) and the library versions.
 """
 from __future__ import annotations
 
@@ -25,6 +26,8 @@ from vit_pytorch import ViT, SimpleViT  # noqa: E402  (the reference)
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+
+from golden_weights import golden_model, state_digest  # noqa: E402  (tests/golden/)
 
 CASES = {
     # BASELINE.json configs[0]: SimpleViT tiny (num_classes / mlp_dim chosen in SURVEY.md 8d)
@@ -89,20 +92,8 @@ def reference_class(kind: str):
 
 
 def make(name: str, spec: dict) -> None:
-    torch.manual_seed(spec["seed"])
     cls = reference_class(spec["kind"])
-    model = cls(**spec["kwargs"]).eval()
-    # bf16-representable parameters; perturb LayerNorm affine params so gamma/beta are actually exercised
-    g = torch.Generator().manual_seed(1000 + spec["seed"])
-    with torch.no_grad():
-        for n, p in model.named_parameters():
-            if p.dim() == 1 and ("norm" in n or n.split(".")[-2] in ("0", "1", "3")) and n.endswith("weight"):
-                p.add_(0.1 * torch.randn(p.shape, generator=g))
-            elif p.dim() == 1 and n.endswith("bias"):
-                p.add_(0.05 * torch.randn(p.shape, generator=g))
-            elif n.endswith("gamma"):                       # per-head q / k RMSNorm scales
-                p.mul_(1.0 + 0.2 * torch.randn(p.shape, generator=g))
-            p.copy_(p.bfloat16().float())
+    model = golden_model(cls, spec["kwargs"], spec["seed"])
     torch.manual_seed(100 + spec["seed"])
     img = torch.randn(spec["batch"], 3, *spec["img"]).bfloat16()
     with torch.inference_mode():
@@ -121,7 +112,8 @@ def make(name: str, spec: dict) -> None:
         "name": name,
         "kind": spec["kind"],
         "kwargs": spec["kwargs"],
-        "state_dict": {k: v.bfloat16() for k, v in model.state_dict().items()},
+        "seed": spec["seed"],
+        "state_digest": state_digest({k: v.bfloat16() for k, v in model.state_dict().items()}),
         "input": img,
         "logits_fp32": logits.clone(),
         "logits_ref_bf16": logits_bf16.float().clone(),
@@ -220,7 +212,122 @@ def make_navit_nested() -> None:
               f"{(bf16.float() - fp32).abs().max():.5f}; {os.path.getsize(path) / 1e6:.2f} MB")
 
 
+def _signature(cls) -> list:
+    import inspect
+    return [(n, p.default) for n, p in inspect.signature(cls.__init__).parameters.items() if n != "self"]
+
+
+def make_reference_surface() -> None:
+    """reference_surface.pt: what the tests used to ask the reference package itself -- constructor signatures, the
+    parameters its constructors draw under a seed (sha256 per tensor, golden_weights.state_digest), its fp32
+    outputs on seeded models, and the values its wrappers (Extractor, Recorder, MAE, DistillWrapper,
+    AcceptVideoWrapper) read from or compute with a ViT."""
+    import importlib
+    from vit_pytorch.na_vit import NaViT as RefNaViT
+    from vit_pytorch.na_vit_nested_tensor import NaViT as RefNestedNaViT
+    from vit_pytorch.recorder import Recorder
+    from vit_pytorch.extractor import Extractor
+    blob = {"init": {}, "signatures": {}, "oracle": {}}
+
+    def init(name, cls, seed, kwargs, buffers=()):
+        torch.manual_seed(seed)
+        m = cls(**kwargs)
+        blob["init"][name] = {"seed": seed, "kwargs": kwargs, "digest": state_digest(m.state_dict()),
+                              "buffers": state_digest({b: getattr(m, b) for b in buffers})}
+        return m
+
+    small = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=2, heads=2, mlp_dim=96, dim_head=32)
+    init("vit", ViT, 123, small)
+    init("simple", SimpleViT, 123, small, buffers=("pos_embedding",))
+    for name, spec in {**CASES2, **CASES3}.items():
+        if spec["kind"] != "vit":
+            init(name, reference_class(spec["kind"]), 123, spec["kwargs"])
+            blob["signatures"][spec["kind"]] = _signature(reference_class(spec["kind"]))
+    init("navit_nested", RefNestedNaViT, 5,
+         dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1, heads=1, mlp_dim=64))
+    blob["signatures"]["na_vit_nested_tensor"] = _signature(RefNestedNaViT)
+
+    # tests/test_oracle.py: seeded reference models and inputs, fp32 logits
+    live = {"vit_11": ("vit", 11), "simple_12": ("simple", 12), "vit_13": ("vit", 13)}
+    for name, (kind, seed) in live.items():
+        kwargs = dict(image_size=64, patch_size=16, num_classes=17, dim=128, depth=2, heads=2, mlp_dim=192)
+        if seed == 13:
+            kwargs["pool"] = "mean"
+        model = init(name, ViT if kind == "vit" else SimpleViT, seed, kwargs).eval()
+        img = torch.randn(3, 3, 64, 64)
+        with torch.inference_mode():
+            blob["oracle"][name] = {"kind": kind, "input": state_digest({"img": img})["img"], "logits": model(img)}
+    vit_b16 = dict(image_size=224, patch_size=16, num_classes=1000, dim=768, depth=12, heads=12, mlp_dim=3072)
+    model = init("vit_b16", ViT, 0, vit_b16).eval()
+    torch.manual_seed(1)
+    img = torch.randn(1, 3, 224, 224)
+    with torch.inference_mode():
+        blob["oracle"]["vit_b16"] = {"kind": "vit", "input": state_digest({"img": img})["img"], "logits": model(img)}
+
+    # tests/test_navit.py: packed NaViT forward on three images
+    kwargs = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1, heads=2, mlp_dim=96, dim_head=32)
+    model = init("navit", RefNaViT, 9, kwargs).eval()
+    imgs = [torch.randn(3, 32, 16), torch.randn(3, 8, 8), torch.randn(3, 24, 32)]
+    with torch.inference_mode():
+        blob["navit"] = {"images": imgs, "logits": model([imgs[:2], imgs[2:]])}
+
+    # Extractor / Recorder (tests/test_dropin.py): embeddings and attention maps of a seeded ViT
+    kwargs = dict(image_size=32, patch_size=8, num_classes=3, dim=32, depth=2, heads=2, mlp_dim=48, dim_head=16)
+    v = init("vit_hooks", ViT, 0, kwargs).eval()
+    img = torch.randn(2, 3, 32, 32)
+    with torch.no_grad():
+        logits, emb = Extractor(v)(img)
+        _, attns = Recorder(v)(img)
+    blob["hooks"] = {"img": img, "logits": logits, "embeddings": emb, "attns": attns}
+
+    # MAE: the encoder members it reads and the encoder call on the unmasked quarter of the tokens
+    kwargs = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=2, heads=2, mlp_dim=96, pool="mean")
+    enc = init("vit_mae", ViT, 0, kwargs).eval()
+    img = torch.randn(3, 3, 32, 32)
+    with torch.no_grad():
+        patches = enc.to_patch_embedding[0](img)
+        tokens = torch.nn.Sequential(*enc.to_patch_embedding[1:])(patches) + enc.pos_embedding
+        torch.manual_seed(2)
+        keep = torch.rand(3, patches.shape[1]).argsort(dim=-1)[:, int(0.75 * patches.shape[1]):]
+        encoded = enc.transformer(tokens[torch.arange(3)[:, None], keep])
+    blob["mae"] = {"img": img, "patches": patches, "tokens": tokens, "keep": keep, "encoded": encoded,
+                   "pixel_values_per_patch": enc.to_patch_embedding[2].weight.shape[-1]}
+
+    # AcceptVideoWrapper: `patch_size`, and the frames of a clip through forward() as one batch
+    kwargs = dict(image_size=32, patch_size=8, num_classes=7, dim=32, depth=1, heads=2, mlp_dim=48, dim_head=16)
+    net = init("vit_video", ViT, 0, kwargs).eval()
+    torch.manual_seed(3)
+    video = torch.randn(2, 3, 4, 32, 32)
+    Wrapper = importlib.import_module("vit_pytorch.accept_video_wrapper").AcceptVideoWrapper
+    with torch.no_grad():
+        frames = net(video.permute(0, 2, 1, 3, 4).reshape(8, 3, 32, 32))
+        wrapped = Wrapper(net, add_time_pos_emb=False)(video)
+    assert torch.allclose(wrapped, frames.reshape(2, 4, 7))
+    blob["video"] = {"video": video, "patch_size": Wrapper(net).patch_size, "frames": frames}
+
+    # DistillWrapper calls teacher(img) under no_grad: fp32 and the reference's own bf16 teacher logits
+    for name, kwargs, shape in (("distill", dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1,
+                                                 heads=2, mlp_dim=96), (2, 3, 32, 32)),
+                                ("distill_gpu", dict(image_size=64, patch_size=8, num_classes=10, dim=128, depth=2,
+                                                     heads=2, mlp_dim=256), (4, 3, 64, 64))):
+        teacher = init(name, ViT, 0, kwargs).eval()
+        torch.manual_seed(4)
+        img = torch.randn(shape).bfloat16()
+        with torch.no_grad():
+            blob[name] = {"img": img, "logits_fp32": teacher(img.float()),
+                          "logits_ref_bf16": teacher.bfloat16()(img).float()}
+
+    blob["versions"] = {"torch": str(torch.__version__), "reference": "vit-pytorch 1.23.6"}
+    path = os.path.join(HERE, "reference_surface.pt")
+    torch.save(blob, path)
+    print(f"reference_surface: {len(blob['init'])} seeded constructors, {len(blob['signatures'])} signatures; "
+          f"{os.path.getsize(path) / 1e6:.2f} MB")
+
+
 if __name__ == "__main__":
+    if len(sys.argv) > 1 and sys.argv[1] == "surface":
+        make_reference_surface()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "navit_nested":
         make_navit_nested()
         sys.exit(0)
@@ -240,3 +347,4 @@ if __name__ == "__main__":
     make_navit()
     make_navit_config5()
     make_navit_nested()
+    make_reference_surface()

@@ -6,10 +6,12 @@ import pytest
 import torch
 from torch import nn
 
-from conftest import import_reference, load_golden, reference_available
+from conftest import load_golden, reference_init, state_digest
 from vit_pytorch_b200 import SimpleViT, ViT
 from vit_pytorch_b200 import simple_vit as sv_mod
 from vit_pytorch_b200 import vit as vit_mod
+
+SURFACE = load_golden("reference_surface")
 
 
 def _build(g):
@@ -121,86 +123,58 @@ def test_hooks_force_the_observable_graph():
     h.remove()
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("kind", ["vit", "simple"])
 def test_same_seed_gives_bit_identical_init(kind):
-    ref = import_reference()
-    kwargs = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=2, heads=2, mlp_dim=96, dim_head=32)
-    torch.manual_seed(123)
-    a = (ref.ViT if kind == "vit" else ref.SimpleViT)(**kwargs)
-    torch.manual_seed(123)
-    b = (ViT if kind == "vit" else SimpleViT)(**kwargs)
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa) == list(sb)
-    for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
+    # reference_init checks every parameter against the digest of the reference constructor under the same seed
+    b = reference_init(kind, ViT if kind == "vit" else SimpleViT)
     if kind == "simple":
-        assert torch.equal(a.pos_embedding, b.pos_embedding)
+        assert state_digest({"pos_embedding": b.pos_embedding}) == SURFACE["init"]["simple"]["buffers"]
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present (GPU box)")
 def test_reference_wrappers_accept_the_dropin():
-    """Recorder / Extractor from the reference operate on our module tree (SURVEY.md 3.4)."""
-    import importlib
-    import_reference()
-    Extractor = importlib.import_module("vit_pytorch.extractor").Extractor
-    v = ViT(image_size=32, patch_size=8, num_classes=3, dim=32, depth=2, heads=2, mlp_dim=48, dim_head=16).eval()
-    logits, emb = Extractor(v)(torch.randn(2, 3, 32, 32))
-    assert logits.shape == (2, 3) and emb.shape == (2, 17, 32)
-
-
-def _pair_with_reference(**kwargs):
-    """Our ViT and the reference's with the same weights (fp32, eval)."""
-    import importlib
-    import_reference()
-    RefViT = importlib.import_module("vit_pytorch.vit").ViT
-    torch.manual_seed(0)
-    ours = ViT(**kwargs).eval()
-    ref = RefViT(**kwargs).eval()
-    ref.load_state_dict(ours.state_dict())
-    return ours, ref
-
-
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present")
-def test_reference_mae_wrapper_runs_on_the_dropin():
-    """MAE (reference mae.py:28-31,50-55,74) reads `to_patch_embedding[0]`, `[1:]`, `[2].weight`, `pos_embedding`,
-    `pool` and calls `encoder.transformer(tokens)` on the unmasked quarter of the tokens: same loss as on the
-    reference's own ViT.  (pool='mean': with the 2-D `pos_embedding` of vit.py:107 the wrapper's `[:, 1:n+1]` slice for
-    pool='cls' -- and SimMIM's, simmim.py:45 -- fails on the reference's own ViT too, so there is nothing to match.)"""
-    import importlib
-    ours, ref = _pair_with_reference(image_size=32, patch_size=8, num_classes=5, dim=64, depth=2, heads=2, mlp_dim=96,
-                                     pool="mean")
-    MAE = importlib.import_module("vit_pytorch.mae").MAE
-    make = lambda enc: MAE(encoder=enc, decoder_dim=32, masking_ratio=0.75, decoder_depth=1, decoder_heads=2,  # noqa
-                           decoder_dim_head=16)
-    torch.manual_seed(1)
-    a = make(ours).eval()
-    b = make(ref).eval()
-    b.load_state_dict(a.state_dict())
-    img = torch.randn(3, 3, 32, 32)
+    """Extractor (reference extractor.py:46-59) hooks `vit.transformer` and returns the logits with the transformer
+    output: on a drop-in with the reference's seeded weights both equal what the reference's Extractor returned on the
+    reference's own ViT."""
+    v = reference_init("vit_hooks", ViT).eval()
+    g = SURFACE["hooks"]
+    seen = []
+    v.transformer.register_forward_hook(lambda m, i, o: seen.append(o))
     with torch.no_grad():
-        torch.manual_seed(2)
-        la = a(img)
-        torch.manual_seed(2)
-        lb = b(img)
-    assert torch.allclose(la, lb, rtol=1e-5, atol=1e-6), (la, lb)
-    a(img).backward()                                # and it trains: gradients reach the encoder through the wrapper
+        logits = v(g["img"])
+    assert torch.allclose(logits, g["logits"], rtol=1e-5, atol=1e-6)
+    assert len(seen) == 1 and torch.allclose(seen[0], g["embeddings"], rtol=1e-5, atol=1e-5)
+
+
+def test_reference_mae_wrapper_runs_on_the_dropin():
+    """MAE (reference mae.py:26-31,46-55,60,74) reads `pos_embedding`, `to_patch_embedding[0]`, `[1:]`, `[2].weight`,
+    `pool` and calls `encoder.transformer(tokens)` on the unmasked quarter of the tokens: every value it reads or gets
+    back equals the reference ViT's (stored from a run of the reference), and gradients reach the encoder through that
+    call.  (pool='mean': with the 2-D `pos_embedding` of vit.py:107 the wrapper's `[:, 1:n+1]` slice for pool='cls'
+    -- and SimMIM's, simmim.py:45 -- fails on the reference's own ViT too, so there is nothing to match.)"""
+    ours = reference_init("vit_mae", ViT).eval()
+    g = SURFACE["mae"]
+    assert ours.pool == "mean" and ours.pos_embedding.shape[-2:] == (16, 64)
+    assert ours.to_patch_embedding[2].weight.shape[-1] == g["pixel_values_per_patch"]
+    with torch.no_grad():
+        patches = ours.to_patch_embedding[0](g["img"])
+        tokens = nn.Sequential(*ours.to_patch_embedding[1:])(patches) + ours.pos_embedding
+        encoded = ours.transformer(tokens[torch.arange(3)[:, None], g["keep"]])
+    assert torch.equal(patches, g["patches"])
+    assert torch.allclose(tokens, g["tokens"], rtol=1e-5, atol=1e-6)
+    assert torch.allclose(encoded, g["encoded"], rtol=1e-5, atol=1e-5), (encoded - g["encoded"]).abs().max()
+    ours.transformer(tokens[:, :4].detach()).sum().backward()     # and it trains through that call
     assert ours.transformer.layers[0][0].to_qkv.weight.grad is not None
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present")
 def test_reference_distill_wrapper_accepts_the_dropin_as_teacher():
-    """DistillWrapper (reference distill.py:104-152) calls `teacher(img)` under no_grad."""
-    import importlib
-    import_reference()
-    distill = importlib.import_module("vit_pytorch.distill")
-    kw = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1, heads=2, mlp_dim=96)
-    torch.manual_seed(0)
-    teacher = ViT(**kw).eval()
-    student = distill.DistillableViT(**kw)
-    loss = distill.DistillWrapper(student=student, teacher=teacher, temperature=3, alpha=0.5)(
-        torch.randn(2, 3, 32, 32), torch.tensor([1, 3]))
-    assert loss.dim() == 0 and torch.isfinite(loss)
+    """DistillWrapper (reference distill.py:139-141) calls `teacher(img)` under no_grad: the drop-in with the
+    reference's seeded weights returns the reference ViT's logits for that call."""
+    teacher = reference_init("distill", ViT).eval()
+    g = SURFACE["distill"]
+    with torch.no_grad():
+        logits = teacher(g["img"].float())
+    assert not logits.requires_grad
+    assert torch.allclose(logits, g["logits_fp32"], rtol=1e-5, atol=1e-6)
 
 
 def test_recorder_and_extractor_twins():
@@ -224,30 +198,20 @@ def test_recorder_and_extractor_twins():
         first = Extractor(v, layer=v.transformer.layers[0][1], layer_save_input=True)
         _, inp = first(img)
         assert isinstance(inp, tuple) and inp[0].shape == (2, 17, 32)
-    if reference_available():
-        import importlib
-        import_reference()
-        RefRecorder = importlib.import_module("vit_pytorch.recorder").Recorder
-        RefViT = importlib.import_module("vit_pytorch.vit").ViT
-        r = RefViT(image_size=32, patch_size=8, num_classes=3, dim=32, depth=2, heads=2, mlp_dim=48, dim_head=16).eval()
-        r.load_state_dict(v.state_dict())
-        with torch.no_grad():
-            _, ref_attns = RefRecorder(r)(img)
-        assert torch.allclose(ref_attns, attns, atol=1e-6)
-
-
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present")
-def test_reference_accept_video_wrapper_runs_on_the_dropin():
-    """AcceptVideoWrapper (reference accept_video_wrapper.py:26-150) reads `image_net.patch_size` and feeds the frames
-    of a clip through `image_net.forward` as one batch: same output as on the reference's own ViT."""
-    import importlib
-    ours, ref = _pair_with_reference(image_size=32, patch_size=8, num_classes=7, dim=32, depth=1, heads=2, mlp_dim=48,
-                                     dim_head=16)
-    Wrapper = importlib.import_module("vit_pytorch.accept_video_wrapper").AcceptVideoWrapper
-    a = Wrapper(ours, add_time_pos_emb=True, time_seq_len=4, dim_emb=7)
-    b = Wrapper(ref, add_time_pos_emb=True, time_seq_len=4, dim_emb=7)
-    b.load_state_dict(a.state_dict())
-    assert a.patch_size == b.patch_size == (8, 8)
-    video = torch.randn(2, 3, 4, 32, 32)
+    # the reference's Recorder on the reference's ViT with the same seeded weights and input
+    assert state_digest(v.state_dict()) == SURFACE["init"]["vit_hooks"]["digest"]
     with torch.no_grad():
-        assert torch.allclose(a(video), b(video), rtol=1e-5, atol=1e-6)
+        _, attns = Recorder(v)(SURFACE["hooks"]["img"])
+    assert torch.allclose(SURFACE["hooks"]["attns"], attns, atol=1e-6)
+
+
+def test_reference_accept_video_wrapper_runs_on_the_dropin():
+    """AcceptVideoWrapper (reference accept_video_wrapper.py:70-76,108) reads `image_net.patch_size` and feeds the
+    frames of a clip through `image_net.forward` as one batch: the drop-in with the reference's seeded weights gives
+    the patch size and the per-frame outputs of the reference's own ViT."""
+    ours = reference_init("vit_video", ViT).eval()
+    g = SURFACE["video"]
+    assert ours.patch_size == g["patch_size"] == (8, 8)
+    with torch.no_grad():
+        frames = ours(g["video"].permute(0, 2, 1, 3, 4).reshape(8, 3, 32, 32))
+    assert torch.allclose(frames, g["frames"], rtol=1e-5, atol=1e-6)

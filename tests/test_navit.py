@@ -2,7 +2,7 @@
 import pytest
 import torch
 
-from conftest import import_reference, load_golden, reference_available
+from conftest import load_golden, reference_init
 from oracle import navit_oracle as NO
 from oracle import vit_oracle as O
 from vit_pytorch_b200.na_vit import NaViT, group_images_by_max_seq_len
@@ -60,24 +60,18 @@ def test_patch_order_is_channel_major():
     assert p[1 * 3 + 2, (2 * 2 + 1) * 2 + 0] == img[2, 1 * 2 + 1, 2 * 2 + 0]
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present (GPU box)")
 def test_same_seed_init_and_live_reference():
-    import importlib
-    import_reference()
-    RefNaViT = importlib.import_module("vit_pytorch.na_vit").NaViT
-    kwargs = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1, heads=2, mlp_dim=96, dim_head=32)
-    torch.manual_seed(9)
-    a = RefNaViT(**kwargs).eval()
-    torch.manual_seed(9)
-    b = NaViT(**kwargs).eval()
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa) == list(sb) and all(torch.equal(sa[k], sb[k]) for k in sa)
-    imgs = [torch.randn(3, 32, 16), torch.randn(3, 8, 8), torch.randn(3, 24, 32)]
+    """Seeded reference NaViT (reference_surface.pt): bit-identical parameters from the same seed, and the drop-in
+    and the oracle reproduce the reference's packed forward of three images."""
+    surface = load_golden("reference_surface")
+    b = reference_init("navit", NaViT).eval()
+    imgs, want = surface["navit"]["images"], surface["navit"]["logits"]
     with torch.inference_mode():
-        want = a([imgs[:2], imgs[2:]])
         got = b([imgs[:2], imgs[2:]])
     assert torch.allclose(got, want, rtol=1e-5, atol=1e-6)
-    assert torch.allclose(NO.navit_forward(O.upcast(sa), kwargs, [imgs[:2], imgs[2:]]), want, rtol=1e-4, atol=1e-5)
+    kwargs = surface["init"]["navit"]["kwargs"]
+    assert torch.allclose(NO.navit_forward(O.upcast(b.state_dict()), kwargs, [imgs[:2], imgs[2:]]), want,
+                          rtol=1e-4, atol=1e-5)
 
 
 def test_varlen_index_arrays_host_logic():

@@ -1,10 +1,12 @@
-"""The oracle (oracle/vit_oracle.py) against outputs of the reference: committed golden fixtures, and -- when the
-reference checkout is present (build container) -- the live reference on fresh seeds."""
+"""The oracle (oracle/vit_oracle.py) against outputs of the reference: committed golden fixtures, and the reference's
+logits on seeded models (tests/golden/reference_surface.pt)."""
 import pytest
 import torch
 
-from conftest import import_reference, load_golden, reference_available
+from conftest import load_golden, reference_init, state_digest
 from oracle import vit_oracle as O
+
+SURFACE = load_golden("reference_surface")
 
 
 def test_oracle_matches_golden(golden):
@@ -65,31 +67,26 @@ def test_flops_formula_matches_baseline_md():
     assert abs(f / 1e9 - 34.943) < 5e-3
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present (GPU box)")
 @pytest.mark.parametrize("kind,seed", [("vit", 11), ("simple", 12), ("vit", 13)])
 def test_oracle_matches_live_reference(kind, seed):
-    ref = import_reference()
-    torch.manual_seed(seed)
-    kwargs = dict(image_size=64, patch_size=16, num_classes=17, dim=128, depth=2, heads=2, mlp_dim=192)
-    if kind == "vit" and seed == 13:
-        kwargs["pool"] = "mean"
-    model = (ref.ViT if kind == "vit" else ref.SimpleViT)(**kwargs).eval()
+    """Seeded reference models on a seeded input (reference_surface.pt): the drop-in's constructor rebuilds the
+    reference's parameters bit for bit, the oracle on them gives the reference's logits."""
+    from vit_pytorch_b200 import SimpleViT, ViT
+    name = f"{kind}_{seed}"
+    model = reference_init(name, ViT if kind == "vit" else SimpleViT)
     img = torch.randn(3, 3, 64, 64)
-    with torch.inference_mode():
-        want = model(img)
-    got = O.forward(kind, O.upcast(model.state_dict()), kwargs, img)
-    assert torch.allclose(got, want, rtol=1e-5, atol=5e-6)
+    want = SURFACE["oracle"][name]
+    assert state_digest({"img": img})["img"] == want["input"]
+    got = O.forward(kind, O.upcast(model.state_dict()), SURFACE["init"][name]["kwargs"], img)
+    assert torch.allclose(got, want["logits"], rtol=1e-5, atol=5e-6)
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference checkout not present (GPU box)")
 def test_oracle_matches_live_reference_vit_b16():
-    ref = import_reference()
-    torch.manual_seed(0)
-    kwargs = dict(image_size=224, patch_size=16, num_classes=1000, dim=768, depth=12, heads=12, mlp_dim=3072)
-    model = ref.ViT(**kwargs).eval()
+    from vit_pytorch_b200 import ViT
+    model = reference_init("vit_b16", ViT)
     torch.manual_seed(1)
     img = torch.randn(1, 3, 224, 224)
-    with torch.inference_mode():
-        want = model(img)
-    got = O.vit_forward(O.upcast(model.state_dict()), kwargs, img)
-    assert torch.allclose(got, want, rtol=1e-4, atol=2e-5), (got - want).abs().max()
+    want = SURFACE["oracle"]["vit_b16"]
+    assert state_digest({"img": img})["img"] == want["input"]
+    got = O.vit_forward(O.upcast(model.state_dict()), SURFACE["init"]["vit_b16"]["kwargs"], img)
+    assert torch.allclose(got, want["logits"], rtol=1e-4, atol=2e-5), (got - want["logits"]).abs().max()

@@ -1,24 +1,19 @@
 """Host-side drop-in contract of the SURVEY.md 8(f3) SimpleViT-family variants and of attention without output
 projection: same state_dict layout, same fp32 values as the UNMODIFIED reference (goldens made by
 tests/golden/make_golden.py round2), same constructor keywords, bit-identical init under one seed.  CPU only."""
-import importlib
 import inspect
 
 import pytest
 import torch
 
-from conftest import import_reference, load_golden, reference_available
+from conftest import load_golden, reference_init
+from golden_weights import dropin_class
+
+SURFACE = load_golden("reference_surface")
 
 VARIANTS = ["simplevit_registers", "simplevit_qknorm", "simplevit_patchdrop", "simplevit_flash",
             "simplevit_1d", "simplevit_3d", "simplevit_3d_pf1"]
 ALL = ["vit_tiny_noproj"] + VARIANTS
-
-
-def dropin_class(kind: str):
-    if kind == "vit":
-        from vit_pytorch_b200 import ViT
-        return ViT
-    return importlib.import_module("vit_pytorch_b200." + kind).SimpleViT
 
 
 @pytest.fixture(params=ALL)
@@ -47,26 +42,12 @@ def test_eager_forward_equals_reference_golden(g):
 
 @pytest.mark.parametrize("name", VARIANTS)
 def test_constructor_keywords_and_same_seed_init_equal_the_reference(name):
-    if not reference_available():
-        pytest.skip("reference checkout not present")
     g = load_golden(name)
-    import_reference()
-    ref_cls = importlib.import_module("vit_pytorch." + g["kind"]).SimpleViT
     our_cls = dropin_class(g["kind"])
-    ps_ref = [p for p in inspect.signature(ref_cls.__init__).parameters if p != "self"]
-    ps_our = [p for p in inspect.signature(our_cls.__init__).parameters if p != "self"]
-    assert ps_ref == ps_our
-    for p in ps_ref:
-        assert inspect.signature(ref_cls.__init__).parameters[p].default == \
-            inspect.signature(our_cls.__init__).parameters[p].default, p
-    torch.manual_seed(123)
-    a = ref_cls(**g["kwargs"])
-    torch.manual_seed(123)
-    b = our_cls(**g["kwargs"])
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa.keys()) == list(sb.keys())
-    for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
+    ps_our = [(p, v.default) for p, v in inspect.signature(our_cls.__init__).parameters.items() if p != "self"]
+    assert ps_our == SURFACE["signatures"][g["kind"]]
+    assert SURFACE["init"][name]["kwargs"] == g["kwargs"]
+    reference_init(name, our_cls)                # parameters drawn under seed 123: bit-identical to the reference's
 
 
 def test_patch_dropout_is_training_only():
@@ -124,23 +105,7 @@ def test_navit_nested_dropin_equals_reference_golden(name):
 
 
 def test_navit_nested_same_seed_init_and_signature_equal_the_reference():
-    if not reference_available():
-        pytest.skip("reference checkout not present")
-    import_reference()
-    ref_cls = importlib.import_module("vit_pytorch.na_vit_nested_tensor").NaViT
     from vit_pytorch_b200.na_vit_nested_tensor import NaViT
-    pr = inspect.signature(ref_cls.__init__).parameters
-    po = inspect.signature(NaViT.__init__).parameters
-    assert list(pr) == list(po)
-    for k in pr:
-        if k != "self":
-            assert pr[k].default == po[k].default, k
-    kw = dict(image_size=32, patch_size=8, num_classes=5, dim=64, depth=1, heads=1, mlp_dim=64)
-    torch.manual_seed(5)
-    a = ref_cls(**kw)
-    torch.manual_seed(5)
-    b = NaViT(**kw)
-    sa, sb = a.state_dict(), b.state_dict()
-    assert list(sa.keys()) == list(sb.keys())
-    for k in sa:
-        assert torch.equal(sa[k], sb[k]), k
+    po = [(p, v.default) for p, v in inspect.signature(NaViT.__init__).parameters.items() if p != "self"]
+    assert po == SURFACE["signatures"]["na_vit_nested_tensor"]
+    reference_init("navit_nested", NaViT)        # parameters drawn under seed 5: bit-identical to the reference's

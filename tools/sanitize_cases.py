@@ -10,6 +10,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from vit_pytorch_b200 import NaViT, SimpleViT, ViT, _lib  # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+from golden_weights import load  # noqa: E402
 which = set(sys.argv[1:]) or {"gemm", "attention", "models", "navit"}
 torch.manual_seed(0)
 dev = "cuda"
@@ -61,7 +63,7 @@ if "attention" in which:
 
 if "models" in which:
     for name in ("simplevit_tiny", "vit_tiny_cls", "vit_tiny_mean_nonsquare"):
-        g = torch.load(os.path.join(ROOT, "tests", "golden", name + ".pt"), weights_only=False)
+        g = load(os.path.join(ROOT, "tests", "golden", name + ".pt"))
         m = (ViT if g["kind"] == "vit" else SimpleViT)(**g["kwargs"]).eval()
         m.load_state_dict(g["state_dict"])
         m = m.to(dev, torch.bfloat16)
